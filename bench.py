@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- IMPALA / V-trace learner frames/sec on synthetic 84x84x4 uint8 observations (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -64,7 +64,14 @@ def parse_args():
     ap.add_argument("--max-seconds", type=float, default=150.0, help="wall-time bound of the reference / cpu legs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-cuda", type=int, default=1, help="also time the reference built with -DUSE_CUDA (info only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed optimizer step of each arm computed to "
+                         "DIR/<arm>_<name>.npy (rank 0; see dump_arrays).  The loop then runs reproducibly, which "
+                         "costs time: the timings of such a run are not benchmark numbers")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def dist_env():
@@ -294,6 +301,63 @@ def parity_rounds(acc, model, pump, rank, world, torch, dist):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 22  # elements; the parameters (1,094,476) stay whole, the 19M-element observation batch is sampled
+
+
+def dump_arrays(arm, res, model):
+    """What the last timed optimizer step of one arm computed, as float32 / float64 arrays (integers and bools
+    converted exactly): every leaf of the learner batch the Batcher delivered for it (`<arm>_batch_<keys>`; a leaf of
+    more than DUMP_SAMPLE elements is reduced to the flattened elements at DUMP_SAMPLE sorted indices drawn by
+    numpy.random.default_rng(0), the same for every run), its loss, and the model parameters after the step
+    (flattened in model.parameters() order).  The synthetic observations, the initial model and the action sampler are
+    seeded and the loop runs reproducibly, so a run with the same arguments computes the same; `<arm>_counters` =
+    (optimizer steps, actor steps, env frames) shows that two runs took the same path."""
+    import numpy as np
+    import torch
+
+    def host(t):
+        t = t.detach()
+        if t.dtype == torch.float64 or (not t.is_floating_point() and t.element_size() > 2):
+            t = t.to(torch.float64)
+        else:
+            t = t.to(torch.float32)
+        a = t.cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        return a
+
+    out = {}
+
+    def walk(name, x):
+        if isinstance(x, dict):
+            for k, v in x.items():
+                walk(f"{name}_{k}", v)
+        elif isinstance(x, (list, tuple)):
+            for i, v in enumerate(x):
+                walk(f"{name}_{i}", v)
+        elif isinstance(x, torch.Tensor):
+            out[name] = host(x)
+
+    walk(f"{arm}_batch", res.last_batch)
+    out[f"{arm}_loss"] = host(res.last_loss)
+    out[f"{arm}_params"] = host(torch.cat([p.detach().reshape(-1) for p in model.parameters()]))
+    out[f"{arm}_counters"] = np.array([res.optimizer_steps, res.actor_steps, res.env_train_steps], dtype=np.float64)
+    return out
+
+
+def write_dump(directory, arrays):
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def nvlink_roofline(tm, world):
     """K-A2 inside the timed region, from the Accumulator's own CUDA events on its reduce stream."""
     red = [t for t, ok in zip(tm["reduce_us"], tm["reduced"]) if ok]
@@ -348,8 +412,16 @@ def run_ours(args):
                 service["fn"]()
                 time.sleep(0.0002)
 
-    flags = impala.Flags(actor_batch_size=args.envs, virtual_batch_size=32 * world, device=device)
+    # --dump-outputs runs the loop reproducibly (see Flags.sync_ticks; fixed cuDNN algorithms instead of autotuned ones)
+    # so that two runs, or two builds, can be compared output for output; its timings are not the benchmark's
+    reproducible = args.dump_outputs is not None
+    dump = reproducible and rank == 0
+    flags = impala.Flags(actor_batch_size=args.envs, virtual_batch_size=32 * world, device=device, keep_last_batch=dump,
+                         sync_ticks=reproducible)
     model, optimizer = impala.make_learner(flags)
+    if reproducible:
+        torch.backends.cudnn.benchmark = False
+        torch.backends.cudnn.deterministic = True
     rpc = api.Rpc()
     rpc.set_name(f"learner{rank}")
     rpc.connect(addr)
@@ -372,6 +444,7 @@ def run_ours(args):
     hbm, peak_kind = measured_peaks()
     K, W, S = args.steps, args.warmup, max(0, args.settle)
     results = {}
+    dumped = {}
     timer = BatchOpTimer(torch, _C.kernel_launches)
 
     def wait_for_full_group():
@@ -451,6 +524,10 @@ def run_ours(args):
         res = impala.run_learner(api, flags, acc, model, optimizer, envs, on_step, max_seconds=3600, group=group,
                                  broker=broker, hooks=timer)
         dbg(f"{mode}: loop finished")
+        if dump:
+            # the loop stopped right after the last timed step: the model still holds its result
+            dumped.update(dump_arrays(mode, res, model))
+            res.last_batch = None
         ms = start_evt.elapsed_time(end_evt)
         wall = (state["t1"] - state["t0"]) * 1e3
         t = torch.tensor([ms, wall], dtype=torch.float64)
@@ -531,10 +608,14 @@ def run_ours(args):
             "optimizer_steps_per_s": {"value": round(K / (v["ms"] / 1e3), 2), "e2e": round(K / (e["ms"] / 1e3), 2)},
             "loop_stats_rank0": {"value": v["loop"], "e2e": e["loop"]},
         }
+        if reproducible:
+            line["reproducible_mode"] = "--dump-outputs: device synchronised every loop iteration, fixed cuDNN algorithms"
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_leg(args)
             if args.ref_cuda:
                 line["reference_cuda_model"] = reference_cuda_leg(args)
+        if dump:
+            write_dump(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     barrier()
     if world > 1:

@@ -128,6 +128,10 @@ class Flags:
     paced_actor: bool = True          # at most ceil(actor steps per learner batch) actor steps between two learner steps
                                       # while learner batches are queued: the GPU sees an even mix instead of bursts of
                                       # ~20 actor steps, so the lock-step of N learners does not wait on one peer's burst
+    keep_last_batch: bool = False     # LearnerResult.last_batch = the learner batch of the latest gradient computation
+    sync_ticks: bool = False          # finish all device work before every loop iteration: which iteration sees a
+                                      # reduction's result then no longer depends on device progress, so the actor /
+                                      # learner interleaving (and with it every result) repeats from run to run
     seed: int = 1234
 
 
@@ -202,6 +206,7 @@ class LearnerResult:
         self.env_train_steps = 0
         self.actor_steps = 0
         self.last_loss = None
+        self.last_batch = None
         self.grad_norm_sum = 0.0
         # where the host thread spends its ticks (wall seconds, counts)
         self.t_learn = self.t_act = self.t_opt = self.t_idle = 0.0
@@ -259,6 +264,8 @@ class LearnerLoop:
     def tick(self):
         """One loop iteration.  Returns True when it performed an optimizer step."""
         flags, acc, model = self.flags, self.acc, self.model
+        if flags.sync_ticks:
+            torch.cuda.synchronize(self.device)
         if _DEBUG and time.time() - self._last_dbg > 5 and hasattr(acc, "debug_state"):
             self._last_dbg = time.time()
             print(f"[dbg pid {os.getpid()}] steps={self.res.optimizer_steps} actor={self.res.actor_steps} "
@@ -293,7 +300,10 @@ class LearnerLoop:
             self.res.t_opt += time.perf_counter() - t_tick
             return True
         if self.learn_size() and acc.wants_gradients():
-            self.res.last_loss = compute_gradients(model, self.learn_get(), flags, self.fused_vtrace)
+            batch = self.learn_get()
+            if flags.keep_last_batch:
+                self.res.last_batch = batch
+            self.res.last_loss = compute_gradients(model, batch, flags, self.fused_vtrace)
             self.res.env_train_steps += flags.unroll_length * flags.batch_size
             acc.reduce_gradients(flags.batch_size)
             self.actor_since_learn = 0

@@ -73,6 +73,7 @@ struct Shared {
   uint64_t size;
   std::atomic<uint64_t> allocated;
   std::atomic<uint32_t> clients, terminate, workerError;
+  std::atomic<uint32_t> errorClaimed;  // the first failing worker writes errorText, then sets workerError
   char errorText[512];
   uint32_t batchSize, numBuffers, numClients;
   ClientIO io[kMaxClients];
@@ -235,7 +236,11 @@ void stepEnv(Shared* sh, size_t bufferIndex, size_t row, WorkerEnv& e, py::objec
       }
     }
   } catch (const std::exception& ex) {
-    if (!sh->workerError.exchange(1)) std::snprintf(sh->errorText, sizeof(sh->errorText), "Error in env: %s", ex.what());
+    if (!sh->errorClaimed.exchange(1)) {
+      // the learner throws errorText as soon as it sees workerError: the text must be complete before the flag is set
+      std::snprintf(sh->errorText, sizeof(sh->errorText), "Error in env: %s", ex.what());
+      sh->workerError.store(1, std::memory_order_release);
+    }
     for (size_t i = 0; i < kMaxClients; ++i) sem_post(&sh->io[i].outSem);
   }
   _exit(0);

@@ -4,7 +4,8 @@ source tree does not.
 
     python tests/golden/make_golden.py            # writes batcher_golden.npz, allreduce_golden.npz, accumulator_golden.npz
 
-Inputs are regenerated from the stored seeds with numpy's PCG64 (stable across versions); outputs are stored verbatim.
+Inputs are regenerated from the stored seeds with numpy's PCG64 (stable across versions); outputs are stored verbatim,
+except the batches of the random Batcher trials (batcher_random_golden.npz), which are stored as digests.
 """
 import os
 import sys
@@ -87,6 +88,45 @@ def make_batcher():
     print("batcher:", len(trials), "trials,", len(out), "arrays")
 
 
+def batcher_random_trials():
+    """(size, dim, shape, n_items) drawn the way the reference's test/unit/test_batcher.py:13-52 draws them."""
+    import random
+    rnd = random.Random(1234)
+    trials = []
+    for _ in range(64):
+        size, dim = rnd.randint(1, 20), rnd.randint(0, 2)
+        dims = rnd.randint(dim + 1, dim + 2)
+        n = rnd.randint(20, 60)
+        shape = [rnd.randint(1, 4) for _ in range(dims)]
+        trials.append((size, dim, shape, n))
+    return trials
+
+
+def make_batcher_random():
+    """Every random trial in both modes: how many batches the reference emits after each item, and a digest of every
+    batch (tests/helpers.digest; the batches themselves would be ~400 KB of random floats)."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from helpers import batcher_random_seed, digest
+    out = {}
+    trials = batcher_random_trials()
+    for ti, (size, dim, shape, n) in enumerate(trials):
+        for mode in ("stack", "cat"):
+            b = moolib.Batcher(size=size, dim=dim)
+            emitted, digests = [], []
+            for j in range(n):
+                getattr(b, mode)(torch.from_numpy(gen_input(batcher_random_seed(ti, mode, j), shape, "f32")))
+                k = 0
+                while not b.empty():
+                    digests.append(digest(b.get().numpy()))
+                    k += 1
+                emitted.append(k)
+            out[f"r{ti}_{mode}_emitted"] = np.array(emitted, dtype=np.int32)
+            out[f"r{ti}_{mode}_digests"] = np.array(digests, dtype="<u8")
+    np.savez_compressed(os.path.join(HERE, "batcher_random_golden.npz"),
+                        trials=np.array([repr(t) for t in trials]), **out)
+    print("batcher_random:", len(trials), "trials x 2 modes")
+
+
 class Peers:
     """N reference Rpc peers + a Broker in this process on loopback (the layout of test/test_reduce.py:97-104)."""
 
@@ -147,6 +187,24 @@ def make_allreduce():
         del peers
     np.savez_compressed(os.path.join(HERE, "allreduce_golden.npz"), cases=np.array(cases), **out)
     print("allreduce:", len(cases), "cases")
+
+
+def make_allreduce_2049():
+    """group.all_reduce of 4 peers on 3 rounds of 2049 floats drawn from default_rng(2026) (odd: vectorised loops end
+    in a partial tail)."""
+    n, numel = 4, 2049
+    peers = Peers(n, 4700, group_name="live")
+    rng = np.random.default_rng(2026)
+    out = {}
+    for rep in range(3):
+        ins = [rng.standard_normal(numel).astype(np.float32) for _ in range(n)]
+        futs = [peers.groups[r].all_reduce(f"live{rep}", torch.from_numpy(ins[r].copy())) for r in range(n)]
+        res = [f.result(30).numpy() for f in futs]
+        assert all(r.tobytes() == res[0].tobytes() for r in res), "reference peers disagree"
+        out[f"rep{rep}"] = res[0].copy()
+        peers.pump()
+    np.savez_compressed(os.path.join(HERE, "allreduce_2049_golden.npz"), n=np.array(n), numel=np.array(numel), **out)
+    print("allreduce_2049: 3 rounds")
 
 
 def make_accumulator():
@@ -301,13 +359,18 @@ def make_vtrace():
 
 
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["batcher", "allreduce", "accumulator", "envpool", "vtrace"]
+    which = sys.argv[1:] or ["batcher", "batcher_random", "allreduce", "allreduce_2049", "accumulator", "envpool",
+                             "vtrace"]
     if "vtrace" in which:
         make_vtrace()
     if "batcher" in which:
         make_batcher()
+    if "batcher_random" in which:
+        make_batcher_random()
     if "allreduce" in which:
         make_allreduce()
+    if "allreduce_2049" in which:
+        make_allreduce_2049()
     if "accumulator" in which:
         make_accumulator()
     if "envpool" in which:

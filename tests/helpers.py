@@ -1,5 +1,6 @@
 """Shared by the CPU and GPU test files: deterministic inputs (identical to tests/golden/make_golden.py)."""
 import ast
+import hashlib
 
 import numpy as np
 
@@ -17,6 +18,17 @@ def gen_input(seed, shape, dt):
 
 def batcher_trials(golden):
     return [ast.literal_eval(str(t)) for t in golden["trials"]]
+
+
+def batcher_random_seed(trial, mode, item):
+    """Input seed of item `item` of random Batcher trial `trial` (tests/golden/batcher_random_golden.npz)."""
+    return 100000 + 200 * trial + 100 * (mode == "cat") + item
+
+
+def digest(a):
+    """64 bits of the SHA-256 of an array's dtype, shape and bytes: stands in for outputs too large to store verbatim."""
+    h = hashlib.sha256(f"{a.dtype.str}{tuple(a.shape)}".encode() + np.ascontiguousarray(a).tobytes())
+    return np.frombuffer(h.digest()[:8], dtype="<u8")[0]
 
 
 def tree_masks(n):
