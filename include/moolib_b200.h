@@ -124,7 +124,8 @@ MB_API int mb_scatter_actions(uint32_t* counters_hostmapped, uint64_t counter_st
                        uint64_t n, mb_stream_t stream);
 
 /* =====================================================================================================
- * HP-A  gradient allreduce over NVLink peer memory (fp32 sum, fixed rank order, fused 1/numGradients scale)
+ * HP-A  gradient allreduce over NVLink peer memory (fp32 sums of fp32 / bf16 / fp16 gradients, fixed rank order,
+ *       fused 1/numGradients scale)
  * ===================================================================================================== */
 
 typedef struct mb_ar_ctx mb_ar_ctx;
@@ -253,6 +254,55 @@ MB_API int mb_ar_result(mb_ar_ctx* ctx, int slot, mb_ar_hdr* sum_out, int* statu
 
 /* Padded flat length (in floats) of a tensor list under the layout rule above. */
 MB_API uint64_t mb_ar_flat_numel(const uint64_t* numel, int ntensors);
+
+/* ---- low-precision gradients (bf16 / fp16), alone or mixed with fp32 in one list ----------------------------------
+ * Element dtypes of the _ex entry points.  For bf16 and fp16 every element is reduced as
+ *     widen each rank's value to fp32;  sum in fp32 in ascending rank order over the ranks with has_grads;
+ *     multiply by the fp32 reciprocal 1.0f/sum(num_gradients) (when scaling);  round ONCE (nearest-even) to the dtype.
+ * All ranks hold identical bits, one-shot and two-shot give identical bits, and a single contributor's result equals
+ * the reference's copy_ + mul_ in the dtype.  The reference instead rounds to the dtype after every tree add
+ * (src/group.h:597-603) and again in mul_ (src/accumulator.cc:442), so it differs in the last bits (DESIGN.md §2). */
+#define MB_DT_F32 0
+#define MB_DT_BF16 1
+#define MB_DT_F16 2
+
+/* One dtype run of the flat layout: bytes [begin, end) hold only tensors of `dtype`. */
+typedef struct mb_ar_segment {
+  uint64_t begin;
+  uint64_t end;
+  int32_t dtype;
+  int32_t reserved;
+} mb_ar_segment;
+
+/* The flat layout of a mixed tensor list, the one rule every _ex call, K-A1 and K-A2 use.  Tensors are grouped by dtype
+ * (fp32, then bf16, then fp16; list order within a group), so each dtype is one contiguous run of 16 B vectors, and every
+ * tensor starts 16 B aligned (padded to 4 fp32 or 8 half-width elements; padding is zero).  For an all-fp32 list the
+ * offsets are exactly those of mb_ar_stage (offset_bytes[i] = 4 * float offset).  Writes offset_bytes[ntensors] (may be
+ * NULL), *total_bytes (may be NULL) and up to 3 non-empty segments (may be NULL).  Returns the number of segments. */
+MB_API int mb_ar_layout(const uint64_t* numel, const int32_t* dtype, int ntensors, uint64_t* offset_bytes,
+                        uint64_t* total_bytes, mb_ar_segment* segments);
+
+/* K-A1 for a mixed list: staging (=|+=) the list in the layout of mb_ar_layout, optionally zeroing the sources.
+ * `+=` rounds in the tensor's dtype, like the reference's add_.  An all-fp32 list runs mb_ar_stage.
+ * (replaces: src/accumulator.cc:941-980 copy_ / add_ for bf16 and fp16 gradients, and :410-418 zero_) */
+MB_API int mb_ar_stage_ex(mb_ar_ctx* ctx, int slot, const void* const* grads, const uint64_t* numel,
+                          const int32_t* dtype, int ntensors, int accumulate, int zero_src, mb_stream_t stream);
+
+/* K-A2 for a mixed list.  `numel`, `dtype`, `ntensors` describe the layout (mb_ar_layout) and are always required;
+ * the result goes to the tensors `dst` (HOST array of device pointers), or, if dst == NULL, to the 16 B-aligned flat
+ * buffer `flat_dst` of exactly flat_bytes == total_bytes in the same layout.  fp32 segments are reduced exactly as
+ * mb_ar_allreduce, bf16 / fp16 segments as stated above; an all-fp32 list runs mb_ar_allreduce itself.
+ * (replaces: src/group.h:570-654,687-787 tree reduce + share of bf16 / fp16 tensors; src/accumulator.cc:433-452) */
+MB_API int mb_ar_allreduce_ex(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, void* const* dst,
+                              const uint64_t* numel, const int32_t* dtype, int ntensors, void* flat_dst,
+                              uint64_t flat_bytes, int scale_by_num_gradients, int algo, uint32_t timeout_ms,
+                              mb_stream_t stream);
+/* K-A0 + K-A2 for a mixed list: mb_ar_reduce_gated with the arguments of mb_ar_allreduce_ex.
+ * (replaces: src/accumulator.cc:1005-1078 startCount + startReduce for bf16 / fp16 models) */
+MB_API int mb_ar_reduce_gated_ex(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, uint64_t min_batch_size,
+                                 void* const* dst, const uint64_t* numel, const int32_t* dtype, int ntensors,
+                                 void* flat_dst, uint64_t flat_bytes, int scale_by_num_gradients, int algo,
+                                 uint32_t timeout_ms, mb_stream_t stream);
 
 /* Host-side abort: makes every in-flight and future barrier wait on this context fail with MB_ETIMEOUT promptly
  * (peer death / regroup, SURVEY.md section 5 "Hook for HP-A").  Cleared by mb_ar_ctx_reset. */

@@ -17,6 +17,7 @@ MB_AR_BUFS_PER_SLOT = 3
 MB_AR_SHORT = 1
 MB_COPY_MAX_INLINE_JOBS = 512
 MB_SRC_UNKNOWN, MB_SRC_DEVICE, MB_SRC_HOST_MAPPED = 0, 1, 2
+MB_DT_F32, MB_DT_BF16, MB_DT_F16 = 0, 1, 2
 
 # every symbol include/moolib_b200.h declares (tests check the .so exports all of them)
 SYMBOLS = [
@@ -26,6 +27,7 @@ SYMBOLS = [
     "mb_ar_ctx_create", "mb_ar_ctx_destroy", "mb_ar_ctx_export", "mb_ar_ctx_import", "mb_ar_ctx_reset",
     "mb_ar_staging", "mb_ar_world", "mb_ar_rank", "mb_ar_stage", "mb_ar_allreduce", "mb_ar_result",
     "mb_ar_flat_numel", "mb_ar_abort", "mb_ar_buffer", "mb_ar_slot_advance", "mb_ar_reduce_gated", "mb_ar_round_times", "mb_vtrace_f32", "mb_u8_to_f32", "mb_ar_xfer_pack", "mb_ar_xfer_unpack", "mb_ar_algo_for",
+    "mb_ar_layout", "mb_ar_stage_ex", "mb_ar_allreduce_ex", "mb_ar_reduce_gated_ex",
 ]
 
 
@@ -47,6 +49,11 @@ class ArHdr(ctypes.Structure):
         ("num_gradients", ctypes.c_uint64), ("num_skipped", ctypes.c_uint64), ("batch_size", ctypes.c_uint64),
         ("has_grads", ctypes.c_uint64),
     ]
+
+
+class ArSegment(ctypes.Structure):
+    _fields_ = [("begin", ctypes.c_uint64), ("end", ctypes.c_uint64), ("dtype", ctypes.c_int32),
+                ("reserved", ctypes.c_int32)]
 
 
 class ArHandle(ctypes.Structure):
@@ -105,6 +112,14 @@ def load():
     L.mb_ar_reduce_gated.argtypes = [vp, ci, ctypes.POINTER(ArHdr), u64, ctypes.POINTER(vp), ctypes.POINTER(u64), ci, vp,
                                      u64, ci, ci, u32, vp]
     L.mb_ar_round_times.argtypes = [vp, ci, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float)]
+    i32p = ctypes.POINTER(ctypes.c_int32)
+    L.mb_ar_layout.argtypes = [ctypes.POINTER(u64), i32p, ci, ctypes.POINTER(u64), ctypes.POINTER(u64),
+                               ctypes.POINTER(ArSegment)]
+    L.mb_ar_stage_ex.argtypes = [vp, ci, ctypes.POINTER(vp), ctypes.POINTER(u64), i32p, ci, ci, ci, vp]
+    L.mb_ar_allreduce_ex.argtypes = [vp, ci, ctypes.POINTER(ArHdr), ctypes.POINTER(vp), ctypes.POINTER(u64), i32p, ci,
+                                     vp, u64, ci, ci, u32, vp]
+    L.mb_ar_reduce_gated_ex.argtypes = [vp, ci, ctypes.POINTER(ArHdr), u64, ctypes.POINTER(vp), ctypes.POINTER(u64),
+                                        i32p, ci, vp, u64, ci, ci, u32, vp]
     _lib = L
     return L
 
@@ -311,6 +326,62 @@ class ArContext:
         ptrs, numel, n = self._lists(tensors)
         return check(self.L.mb_ar_xfer_unpack(self._ctx, src_rank, ptrs, numel, n, _stream_ptr(stream)))
 
+    # ---- mixed-dtype lists (fp32 / bf16 / fp16): the _ex entry points, layout of mb_ar_layout ----
+    @staticmethod
+    def _lists_ex(tensors):
+        n = len(tensors)
+        ptrs = (ctypes.c_void_p * n)(*[t.data_ptr() for t in tensors])
+        numel = (ctypes.c_uint64 * n)(*[t.numel() for t in tensors])
+        dts = (ctypes.c_int32 * n)(*[dtype_code(t.dtype) for t in tensors])
+        return ptrs, numel, dts, n
+
+    def stage_ex(self, tensors, slot=0, accumulate=False, zero_src=False, stream=None):
+        ptrs, numel, dts, n = self._lists_ex(tensors)
+        return check(self.L.mb_ar_stage_ex(self._ctx, slot, ptrs, numel, dts, n, int(accumulate), int(zero_src),
+                                           _stream_ptr(stream)))
+
+    def _reduce_ex(self, gated, min_batch, tensors, flat_dst, hdr, slot, scale, algo, timeout_ms, stream):
+        """tensors: the destination list, or (flat_dst given) tensors / (numel, torch dtype) pairs describing the
+        layout of the flat uint8 result buffer."""
+        h = ArHdr(*hdr)
+        if flat_dst is None:
+            ptrs, numel, dts, n = self._lists_ex(tensors)
+            flat_ptr, flat_bytes = None, 0
+        else:
+            desc = [(t.numel(), t.dtype) if hasattr(t, "numel") else t for t in tensors]
+            n = len(desc)
+            ptrs = None
+            numel = (ctypes.c_uint64 * n)(*[m for m, _ in desc])
+            dts = (ctypes.c_int32 * n)(*[dtype_code(d) for _, d in desc])
+            flat_ptr, flat_bytes = flat_dst.data_ptr(), flat_dst.numel() * flat_dst.element_size()
+        if gated:
+            return check(self.L.mb_ar_reduce_gated_ex(self._ctx, slot, ctypes.byref(h), min_batch, ptrs, numel, dts, n,
+                                                      flat_ptr, flat_bytes, int(scale), algo, timeout_ms,
+                                                      _stream_ptr(stream)))
+        return check(self.L.mb_ar_allreduce_ex(self._ctx, slot, ctypes.byref(h), ptrs, numel, dts, n, flat_ptr,
+                                               flat_bytes, int(scale), algo, timeout_ms, _stream_ptr(stream)))
+
+    def allreduce_ex(self, tensors, flat_dst=None, hdr=(1, 0, 1, 1), slot=0, scale=True, algo=MB_AR_ALGO_AUTO,
+                     timeout_ms=30000, stream=None):
+        return self._reduce_ex(False, 0, tensors, flat_dst, hdr, slot, scale, algo, timeout_ms, stream)
+
+    def reduce_gated_ex(self, min_batch, tensors, flat_dst=None, hdr=(1, 0, 1, 1), slot=0, scale=True,
+                        algo=MB_AR_ALGO_AUTO, timeout_ms=30000, stream=None):
+        return self._reduce_ex(True, min_batch, tensors, flat_dst, hdr, slot, scale, algo, timeout_ms, stream)
+
+    def buffer_bytes(self, nbytes, slot=0, ahead=0):
+        """Like buffer(), as a flat uint8 tensor of `nbytes` (view it per tensor with layout() offsets)."""
+        import torch
+
+        class _Mem:
+            pass
+
+        m = _Mem()
+        m.__cuda_array_interface__ = {"shape": (int(nbytes),), "typestr": "|u1", "version": 3,
+                                      "data": (int(self.buffer_ptr(slot, ahead)), False)}
+        with torch.cuda.device(self.device):
+            return torch.as_tensor(m, device=f"cuda:{self.device}")
+
     def result(self, slot=0):
         h = ArHdr()
         st = ctypes.c_int()
@@ -321,3 +392,25 @@ class ArContext:
 def flat_numel(numels):
     arr = (ctypes.c_uint64 * len(numels))(*numels)
     return load().mb_ar_flat_numel(arr, len(numels))
+
+
+def dtype_code(dt):
+    """MB_DT_* of a torch dtype (or of the strings 'f32', 'bf16', 'f16')."""
+    name = str(dt).replace("torch.", "")
+    codes = {"float32": MB_DT_F32, "f32": MB_DT_F32, "bfloat16": MB_DT_BF16, "bf16": MB_DT_BF16,
+             "float16": MB_DT_F16, "f16": MB_DT_F16}
+    if name not in codes:
+        raise ValueError(f"unsupported allreduce dtype {dt}; supported: float32, bfloat16, float16")
+    return codes[name]
+
+
+def layout(numels, dtypes):
+    """mb_ar_layout: (per-tensor byte offsets, total bytes, [(begin, end, MB_DT_*) per dtype segment])."""
+    n = len(numels)
+    nm = (ctypes.c_uint64 * max(n, 1))(*numels)
+    dt = (ctypes.c_int32 * max(n, 1))(*[dtype_code(d) if not isinstance(d, int) else d for d in dtypes])
+    off = (ctypes.c_uint64 * max(n, 1))()
+    total = ctypes.c_uint64()
+    segs = (ArSegment * 3)()
+    nseg = check(load().mb_ar_layout(nm, dt, n, off, ctypes.byref(total), segs))
+    return list(off)[:n], total.value, [(segs[k].begin, segs[k].end, segs[k].dtype) for k in range(nseg)]

@@ -42,7 +42,7 @@ struct ReduceSlot {
   cudaEvent_t event = nullptr;             // device path: completion of the K-A2 launch
   cudaEvent_t staged = nullptr;            // device path: this slot's gradients are complete (compute stream)
   bool kernelInFlight = false;
-  float* resultBase = nullptr;             // device gate: where K-A2 leaves the averaged gradients (flat layout)
+  void* resultBase = nullptr;              // device gate: where K-A2 leaves the averaged gradients (flat layout)
   bool gated = false;                      // the in-flight launch is K-A0 + K-A2 (mb_ar_reduce_gated)
   Clock::time_point reduceStart;
   ~ReduceSlot() {
@@ -146,10 +146,11 @@ class Accumulator {
     if (gradsOnCuda_) {
       for (auto& p : params_) {
         if (!p.requires_grad()) continue;
-        if (!p.is_cuda() || p.get_device() != device_ || p.scalar_type() != torch::kFloat32)
+        if (!p.is_cuda() || p.get_device() != device_ || dtypeCode(p.scalar_type()) < 0)
           throw std::runtime_error(
-              "moolib_b200.Accumulator: CUDA parameters must all be float32 on one device (the NVLink allreduce sums "
-              "fp32 like the reference's ATen add)");
+              "moolib_b200.Accumulator: CUDA parameters must all be on one device and of dtype float32, bfloat16 or "
+              "float16 (mixed is fine); got " + std::string(c10::toString(p.scalar_type())) + " on " +
+              p.device().str());
       }
     }
     ensureGrads();
@@ -231,8 +232,8 @@ class Accumulator {
         g = torch::zeros_like(p);
         p.mutable_grad() = g;
       }
-      if (gradsOnCuda_ && (!g.is_contiguous() || g.scalar_type() != torch::kFloat32)) {
-        g = g.contiguous().to(torch::kFloat32);
+      if (gradsOnCuda_ && (!g.is_contiguous() || g.scalar_type() != p.scalar_type())) {
+        g = g.contiguous().to(p.scalar_type());
         p.mutable_grad() = g;
       }
       r.push_back(g);
@@ -263,7 +264,7 @@ class Accumulator {
       if (gradsAre(av) || (appliedBase_ && gradsAre(viewsOf(appliedBase_)))) {
         // .grad shows an applied result (or is already accumulating): (back) to the accumulation buffer, zero-filled by
         // ONE memset of the flat buffer (reference: 36 zero_ launches, src/accumulator.cc:410-418)
-        cudaMemsetAsync(av.base, 0, (size_t)arena_->total * 4, c10::cuda::getCurrentCUDAStream(device_).stream());
+        cudaMemsetAsync(av.base, 0, (size_t)arena_->total, c10::cuda::getCurrentCUDAStream(device_).stream());
         pointGradsAt(av);
       } else {
         actuallyZeroGradients();
@@ -276,45 +277,52 @@ class Accumulator {
 
   // ---- gradient arena (device gate path): .grad tensors are views into the symmetric ring / the result buffers ----
   struct GradViews {
-    float* base = nullptr;
-    torch::Tensor flat;
+    void* base = nullptr;
     std::vector<torch::Tensor> v;  // one per parameter that requires grad, same order as ensureGrads()
   };
   struct GradArena {
-    std::vector<int64_t> numel, off;  // floats; off = flat layout of mb_ar_stage (each tensor starts 16 B aligned)
+    std::vector<uint64_t> numel, off;  // off: bytes, the flat layout of mb_ar_layout (dtype runs, 16 B aligned tensors)
+    std::vector<int32_t> dtype;        // MB_DT_*
+    std::vector<c10::ScalarType> type;
     std::vector<std::vector<int64_t>> sizes;
-    int64_t total = 0;                // padded floats
-    std::map<float*, GradViews> views;
+    int64_t total = 0;                 // padded bytes
+    std::map<void*, GradViews> views;
     std::vector<torch::Tensor> result;  // per slot: where K-A2 writes (local memory, flat layout)
   };
 
   GradArena& arena() {
     if (!arena_) {
       arena_ = std::make_unique<GradArena>();
-      int64_t off = 0;
       for (auto& p : params_) {
         if (!p.requires_grad()) continue;
-        arena_->numel.push_back(p.numel());
-        arena_->off.push_back(off);
+        arena_->numel.push_back((uint64_t)p.numel());
+        arena_->dtype.push_back(dtypeCode(p.scalar_type()));
+        arena_->type.push_back(p.scalar_type());
         arena_->sizes.emplace_back(p.sizes().begin(), p.sizes().end());
-        off += (p.numel() + 3) & ~int64_t(3);
       }
-      arena_->total = off;
+      arena_->off.resize(arena_->numel.size());
+      uint64_t total = 0;
+      if (!arena_->numel.empty())
+        check(mb_ar_layout(arena_->numel.data(), arena_->dtype.data(), (int)arena_->numel.size(), arena_->off.data(),
+                           &total, nullptr),
+              "mb_ar_layout");
+      arena_->total = (int64_t)total;
       c10::cuda::CUDAGuard dg(device_);
       for (size_t i = 0; i < slots_.size(); ++i)
-        arena_->result.push_back(torch::empty({std::max<int64_t>(off, 4)}, torch::dtype(torch::kFloat32).device(torch::kCUDA, device_)));
+        arena_->result.push_back(torch::empty({std::max<int64_t>(arena_->total, 16)}, torch::dtype(torch::kUInt8).device(torch::kCUDA, device_)));
     }
     return *arena_;
   }
 
-  GradViews& viewsOf(float* base) {
+  GradViews& viewsOf(void* base) {
     GradArena& a = arena();
     auto it = a.views.find(base);
     if (it != a.views.end()) return it->second;
     GradViews& gv = a.views[base];
     gv.base = base;
-    gv.flat = torch::from_blob(base, {std::max<int64_t>(a.total, 1)}, torch::dtype(torch::kFloat32).device(torch::kCUDA, device_));
-    for (size_t i = 0; i < a.numel.size(); ++i) gv.v.push_back(gv.flat.narrow(0, a.off[i], a.numel[i]).view(a.sizes[i]));
+    for (size_t i = 0; i < a.numel.size(); ++i)
+      gv.v.push_back(torch::from_blob(static_cast<char*>(base) + a.off[i], a.sizes[i],
+                                      torch::dtype(a.type[i]).device(torch::kCUDA, device_)));
     return gv;
   }
 
@@ -323,7 +331,8 @@ class Accumulator {
     for (auto& p : params_) {
       if (!p.requires_grad()) continue;
       const torch::Tensor& g = p.grad();
-      if (!g.defined() || g.data_ptr() != gv.v[i].data_ptr() || g.scalar_type() != torch::kFloat32 || !g.is_contiguous())
+      if (!g.defined() || g.data_ptr() != gv.v[i].data_ptr() || g.scalar_type() != gv.v[i].scalar_type() ||
+          !g.is_contiguous())
         return false;
       ++i;
     }
@@ -344,16 +353,14 @@ class Accumulator {
   }
   // Where the next contribution for slot j is accumulated: the slot's staging itself while it is empty (zero-copy: the
   // peers will read exactly what backward() wrote), else the next ring buffer (folded in by K-A1).
-  float* accumBase(size_t j) {
-    return static_cast<float*>(mb_ar_buffer(reducer()->ctx(), (int)j, slotHoldsData(j) ? 1 : 0));
-  }
+  void* accumBase(size_t j) { return mb_ar_buffer(reducer()->ctx(), (int)j, slotHoldsData(j) ? 1 : 0); }
 
   // Point .grad at the accumulation buffer of the slot that the next reduce_gradients() call fills.
   void repointForAccumulation() {
     c10::cuda::CUDAGuard dg(device_);
     GradViews& av = viewsOf(accumBase(nextIndex_));
     if (gradsAre(av)) return;  // already there (and clean: K-A1 zeroes its sources)
-    cudaMemsetAsync(av.base, 0, (size_t)arena().total * 4, c10::cuda::getCurrentCUDAStream(device_).stream());
+    cudaMemsetAsync(av.base, 0, (size_t)arena().total, c10::cuda::getCurrentCUDAStream(device_).stream());
     pointGradsAt(av);
   }
 
@@ -380,8 +387,29 @@ class Accumulator {
 
   uint64_t flatBytes(const std::vector<torch::Tensor>& gs) {
     std::vector<uint64_t> n;
-    for (auto& g : gs) n.push_back((uint64_t)g.numel());
-    return mb_ar_flat_numel(n.data(), (int)n.size()) * 4;
+    std::vector<int32_t> d;
+    for (auto& g : gs) {
+      n.push_back((uint64_t)g.numel());
+      d.push_back(dtypeCode(g.scalar_type()));
+    }
+    uint64_t total = 0;
+    if (!n.empty()) check(mb_ar_layout(n.data(), d.data(), (int)n.size(), nullptr, &total, nullptr), "mb_ar_layout");
+    return total;
+  }
+  // (pointers, numel, MB_DT_*) of a gradient list for the _ex entry points
+  struct ListEx {
+    std::vector<void*> ptrs;
+    std::vector<uint64_t> numel;
+    std::vector<int32_t> dtype;
+  };
+  static ListEx listEx(const std::vector<torch::Tensor>& gs) {
+    ListEx l;
+    for (auto& g : gs) {
+      l.ptrs.push_back(g.data_ptr());
+      l.numel.push_back((uint64_t)g.numel());
+      l.dtype.push_back(dtypeCode(g.scalar_type()));
+    }
+    return l;
   }
 
   std::shared_ptr<DeviceReducer> reducer() {
@@ -424,19 +452,14 @@ class Accumulator {
       const bool add = target->data.has_grads != 0;
       if (gradsOnCuda_) {
         c10::cuda::CUDAGuard dg(device_);
-        const bool zeroCopy = deviceGate() && !add &&
-                              gradsAre(viewsOf(static_cast<float*>(mb_ar_buffer(reducer()->ctx(), (int)index, 0))));
+        const bool zeroCopy = deviceGate() && !add && gradsAre(viewsOf(mb_ar_buffer(reducer()->ctx(), (int)index, 0)));
         if (!zeroCopy) {
           // K-A1: staging (=|+=) grads and grads <- 0 in one launch, ordered after backward() on the current stream
           // (a user-assigned .grad, or another local contribution while the gate is still closed)
-          std::vector<const float*> ptrs;
-          std::vector<uint64_t> numel;
-          for (auto& g : gs) {
-            ptrs.push_back(g.data_ptr<float>());
-            numel.push_back((uint64_t)g.numel());
-          }
-          launch_counter() += check(mb_ar_stage(reducer()->ctx(), (int)index, ptrs.data(), numel.data(), (int)gs.size(),
-                                                add ? 1 : 0, /*zero_src=*/1, current_stream(device_)),
+          ListEx l = listEx(gs);
+          launch_counter() += check(mb_ar_stage_ex(reducer()->ctx(), (int)index, l.ptrs.data(), l.numel.data(),
+                                                   l.dtype.data(), (int)gs.size(), add ? 1 : 0, /*zero_src=*/1,
+                                                   current_stream(device_)),
                                     "Accumulator.reduce_gradients");
           ++stageLaunches_;
         } else {
@@ -499,13 +522,15 @@ class Accumulator {
     // Two-shot (large gradient sets, N > 2): its all-gather leaves the averaged gradients in every rank's staging
     // buffer, so the result is consumed IN PLACE (.grad will point at this ring position) and the kernel skips its
     // final local copy.  One-shot writes the slot's separate result buffer (peers are still reading the staging).
-    const int algo = mb_ar_algo_for(reducer()->ctx(), (uint64_t)a.total * 4);
-    target->resultBase = algo == MB_AR_ALGO_TWOSHOT ? static_cast<float*>(mb_ar_buffer(reducer()->ctx(), (int)target->index, 0))
-                                                    : a.result[target->index].data_ptr<float>();
+    const int algo = mb_ar_algo_for(reducer()->ctx(), (uint64_t)a.total);
+    target->resultBase = algo == MB_AR_ALGO_TWOSHOT ? mb_ar_buffer(reducer()->ctx(), (int)target->index, 0)
+                                                    : a.result[target->index].data_ptr();
+    // an all-fp32 model runs exactly mb_ar_reduce_gated (flat destination of a.total / 4 floats)
     launch_counter() += check(
-        mb_ar_reduce_gated(reducer()->ctx(), (int)target->index, &target->data, virtualBatchSize_, nullptr, nullptr, 0,
-                           target->resultBase, (uint64_t)a.total, /*scale=*/1, algo,
-                           (uint32_t)(parts_.rpc->getTimeout() * 1000), static_cast<mb_stream_t>(stream)),
+        mb_ar_reduce_gated_ex(reducer()->ctx(), (int)target->index, &target->data, virtualBatchSize_, nullptr,
+                              a.numel.data(), a.dtype.data(), (int)a.numel.size(), target->resultBase,
+                              (uint64_t)a.total, /*scale=*/1, algo, (uint32_t)(parts_.rpc->getTimeout() * 1000),
+                              static_cast<mb_stream_t>(stream)),
         "Accumulator gated allreduce");
     cudaEventRecord(target->event, stream);
     target->kernelInFlight = true;
@@ -538,12 +563,7 @@ class Accumulator {
     torch::NoGradGuard ng;
     if (gradsOnCuda_) {
       auto gs = ensureGrads();
-      std::vector<float*> ptrs;
-      std::vector<uint64_t> numel;
-      for (auto& g : gs) {
-        ptrs.push_back(g.data_ptr<float>());
-        numel.push_back((uint64_t)g.numel());
-      }
+      ListEx l = listEx(gs);
       c10::cuda::CUDAGuard dg(device_);
       // Host-counted path: K-A2 (with its in-kernel barrier) writes the .grad tensors themselves.  Safe: every backward
       // pass that contributed was followed by its stage kernel in the same reduce_gradients() call, no new backward is
@@ -553,9 +573,9 @@ class Accumulator {
       if (target->staged) cudaStreamWaitEvent(stream, target->staged, 0);
       // K-A2: barrier + P2P reduce + 1/numGradients scale + scatter into the .grad tensors, one launch
       launch_counter() += check(
-          mb_ar_allreduce(reducer()->ctx(), (int)target->index, &target->data, ptrs.data(), numel.data(), (int)gs.size(),
-                          nullptr, 0, /*scale=*/1, MB_AR_ALGO_AUTO, (uint32_t)(parts_.rpc->getTimeout() * 1000),
-                          static_cast<mb_stream_t>(stream)),
+          mb_ar_allreduce_ex(reducer()->ctx(), (int)target->index, &target->data, l.ptrs.data(), l.numel.data(),
+                             l.dtype.data(), (int)gs.size(), nullptr, 0, /*scale=*/1, MB_AR_ALGO_AUTO,
+                             (uint32_t)(parts_.rpc->getTimeout() * 1000), static_cast<mb_stream_t>(stream)),
           "Accumulator allreduce");
       if (!target->event) cudaEventCreateWithFlags(&target->event, cudaEventDisableTiming);
       cudaEventRecord(target->event, stream);
@@ -1193,7 +1213,7 @@ class Accumulator {
     d["gate_us"] = gate;      // K-A0: includes the wait for the slowest peer
     d["reduce_us"] = red;     // K-A2: the data movement
     d["reduced"] = ok;        // false: the gate stayed shut (short batch), K-A2 returned at once
-    d["bytes"] = arena_ ? (int64_t)arena_->total * 4 : (int64_t)0;
+    d["bytes"] = arena_ ? (int64_t)arena_->total : (int64_t)0;
     d["world"] = reducer_ ? reducer_->world() : 0;
     d["stage_launches"] = stageLaunches_;
     d["zero_copy_rounds"] = zeroCopyRounds_;
@@ -1234,7 +1254,7 @@ class Accumulator {
   Clock::time_point deferredRequestSince_{}, epochStart_ = Clock::now();
   uint64_t nvlinkPublishes_ = 0, nvlinkFetches_ = 0;
   std::unique_ptr<GradArena> arena_;
-  float* appliedBase_ = nullptr;  // the buffer of the applied result that .grad currently shows (null: none)
+  void* appliedBase_ = nullptr;   // the buffer of the applied result that .grad currently shows (null: none)
   struct RoundTiming {
     float gateUs, reduceUs;
     bool reduced;

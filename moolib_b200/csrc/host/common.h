@@ -28,6 +28,16 @@ inline int check(int rc, const char* what) {
   return rc;
 }
 
+// MB_DT_* of a gradient dtype the NVLink allreduce reduces (float32, bfloat16, float16), -1 for any other
+inline int32_t dtypeCode(c10::ScalarType t) {
+  switch (t) {
+    case c10::ScalarType::Float: return MB_DT_F32;
+    case c10::ScalarType::BFloat16: return MB_DT_BF16;
+    case c10::ScalarType::Half: return MB_DT_F16;
+    default: return -1;
+  }
+}
+
 inline mb_stream_t current_stream(int device) {
   return static_cast<mb_stream_t>(c10::cuda::getCurrentCUDAStream(device).stream());
 }

@@ -245,19 +245,30 @@ struct TensorReduceOp {
         }
         c10::cuda::CUDAGuard dg(reducer->device());
         flat = tensor.is_contiguous() ? tensor : tensor.contiguous();
-        const float* src = flat.data_ptr<float>();
         uint64_t numel = (uint64_t)flat.numel();
         // Own stream per operation name: a gate that waits for the peers must not block the caller's stream, nor sit
         // in front of another operation's gate (two names started in opposite orders on two ranks would deadlock).
         cudaStream_t side = reducer->stream();
         if (ready) cudaStreamWaitEvent(side, ready, 0);
         mb_stream_t s = static_cast<mb_stream_t>(side);
-        launch_counter() += check(mb_ar_stage(reducer->ctx(), 0, &src, &numel, 1, 0, 0, s), "mb_ar_stage");
         mb_ar_hdr hdr{1, 0, 1, 1};
-        launch_counter() += check(mb_ar_reduce_gated(reducer->ctx(), 0, &hdr, /*min_batch=*/0, nullptr, nullptr, 0,
-                                                     flat.data_ptr<float>(), numel, /*scale=*/0, MB_AR_ALGO_AUTO,
-                                                     (uint32_t)(service->rpc()->getTimeout() * 1000), s),
-                                  "mb_ar_reduce_gated");
+        const uint32_t timeoutMs = (uint32_t)(service->rpc()->getTimeout() * 1000);
+        if (flat.scalar_type() == torch::kFloat32) {
+          const float* src = flat.data_ptr<float>();
+          launch_counter() += check(mb_ar_stage(reducer->ctx(), 0, &src, &numel, 1, 0, 0, s), "mb_ar_stage");
+          launch_counter() += check(mb_ar_reduce_gated(reducer->ctx(), 0, &hdr, /*min_batch=*/0, nullptr, nullptr, 0,
+                                                       flat.data_ptr<float>(), numel, /*scale=*/0, MB_AR_ALGO_AUTO,
+                                                       timeoutMs, s),
+                                    "mb_ar_reduce_gated");
+        } else {
+          // bf16 / fp16: widened to fp32, summed in rank order, rounded once (mb_ar_reduce_gated_ex)
+          void* ptr = flat.data_ptr();
+          const int32_t dt = dtypeCode(flat.scalar_type());
+          launch_counter() += check(mb_ar_stage_ex(reducer->ctx(), 0, &ptr, &numel, &dt, 1, 0, 0, s), "mb_ar_stage_ex");
+          launch_counter() += check(mb_ar_reduce_gated_ex(reducer->ctx(), 0, &hdr, /*min_batch=*/0, &ptr, &numel, &dt,
+                                                          1, nullptr, 0, /*scale=*/0, MB_AR_ALGO_AUTO, timeoutMs, s),
+                                    "mb_ar_reduce_gated_ex");
+        }
         if (cudaEventCreateWithFlags(&event, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventRecord(event, side) != cudaSuccess)
           return fail("moolib_b200: cudaEventRecord failed");
@@ -290,8 +301,8 @@ struct TensorReduceOp {
 
 std::shared_ptr<PyFuture> DeviceReducerSet::allReduceTensor(const std::string& name, torch::Tensor t,
                                                             py::object pyTensor) {
-  if (t.scalar_type() != torch::kFloat32)
-    throw std::runtime_error("moolib_b200: all_reduce on CUDA tensors supports float32 (the gradient dtype); got " +
+  if (dtypeCode(t.scalar_type()) < 0)
+    throw std::runtime_error("moolib_b200: all_reduce on CUDA tensors supports float32, bfloat16 and float16; got " +
                              std::string(c10::toString(t.scalar_type())));
   int device = t.get_device();
   auto op = std::make_shared<TensorReduceOp>(c10::cuda::getCurrentCUDAStream(device));
@@ -314,7 +325,7 @@ std::shared_ptr<PyFuture> DeviceReducerSet::allReduceTensor(const std::string& n
   }
   // at most one operation per name is in flight (GroupService rejects "all-reduce twice concurrently"); the name is
   // part of the context key so that differently named operations never share epochs
-  op->reducer = get("ar:" + name, device, sizeClass((uint64_t)t.numel() * 4 + 64), 1);
+  op->reducer = get("ar:" + name, device, sizeClass((uint64_t)t.numel() * t.element_size() + 64), 1);
   {
     std::lock_guard<std::mutex> l(mu_);
     auto& slot = inflight_[name];

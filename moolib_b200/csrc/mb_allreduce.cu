@@ -20,6 +20,8 @@
 // src/group.h:570-654,687-787 (tree reduce + share), src/accumulator.cc:425-452 (copy_ + mul_(1.0f/numGradients)).
 #include "mb_common.cuh"
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <unistd.h>
 
 #include <algorithm>
@@ -128,6 +130,7 @@ struct mb_ar_ctx {
   bool ev_valid[MB_AR_MAX_SLOTS] = {};
   mb::TensorEnt* tab_dev[2] = {nullptr, nullptr};  // 0: stage sources, 1: allreduce destinations
   std::vector<mb::TensorEnt> tab_host[2];
+  bool tab_bytes[2] = {false, false};  // the table holds byte entries (mixed-dtype lists), see SegInfo
   std::mutex mu;
 };
 
@@ -727,6 +730,369 @@ ArKernel kernel_for(int world, bool twoshot, int want_unroll, int* unroll_out) {
   return nullptr;
 }
 
+// ---- mixed-dtype lists (bf16 / fp16 segments) ---------------------------------------------------------------------
+// The 16 B vector stays the unit of every load and store; only the arithmetic on a vector depends on the dtype run
+// (segment) it lies in.  fp32 vectors are reduced exactly as above; a half-width vector is widened to 8 fp32 lanes,
+// summed with __fadd_rn in rank order, scaled with __fmul_rn and rounded once (cvt.rn.{bf16,f16}x2.f32).  The tensor
+// table of these kernels is in BYTES: TensorEnt.off = byte offset / 4 (so load_table's >> 2 still yields the first
+// vector) and TensorEnt.numel = byte length.  All-fp32 lists never reach them (the _ex entry points route those to the
+// kernels above).
+
+struct SegInfo {
+  uint64_t end[3];  // cumulative end of each segment in 16 B vectors (unused: ~0)
+  int32_t dt[3];
+};
+
+struct ArSegParams {
+  ArParams b;
+  SegInfo seg;
+};
+
+struct StageSegParams {
+  StageParams b;
+  SegInfo seg;
+};
+
+__device__ __forceinline__ int seg_dtype(const SegInfo& s, uint64_t v) {
+  return v < s.end[0] ? s.dt[0] : v < s.end[1] ? s.dt[1] : s.dt[2];
+}
+
+__device__ __forceinline__ uint4 ld_peer_u4(const uint4* p) {
+  const float4 f = ld_peer_f4(reinterpret_cast<const float*>(p));
+  return make_uint4(__float_as_uint(f.x), __float_as_uint(f.y), __float_as_uint(f.z), __float_as_uint(f.w));
+}
+__device__ __forceinline__ void st_u4(uint4* p, const uint4& v) {
+  st_f4(reinterpret_cast<float*>(p),
+        make_float4(__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w)));
+}
+
+// 16 B <-> 8 fp32 lanes (half-width dtypes): bf16 widens with a shift, fp16 with cvt.f32.f16 (both exact)
+__device__ __forceinline__ void widen8(int dt, const uint4& x, float (&f)[8]) {
+  const uint32_t w[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    if (dt == MB_DT_BF16) {
+      f[2 * i] = __uint_as_float(w[i] << 16);
+      f[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+    } else {
+      __half2_raw r;
+      r.x = (unsigned short)(w[i] & 0xffffu);
+      r.y = (unsigned short)(w[i] >> 16);
+      const float2 t = __half22float2(__half2(r));
+      f[2 * i] = t.x;
+      f[2 * i + 1] = t.y;
+    }
+  }
+}
+__device__ __forceinline__ uint4 narrow8(int dt, const float (&f)[8]) {
+  uint32_t w[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    if (dt == MB_DT_BF16) {
+      const __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);  // cvt.rn.bf16x2.f32
+      w[i] = *reinterpret_cast<const uint32_t*>(&h);
+    } else {
+      const __half2 h = __floats2half2_rn(f[2 * i], f[2 * i + 1]);  // cvt.rn.f16x2.f32
+      w[i] = *reinterpret_cast<const uint32_t*>(&h);
+    }
+  }
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+// Sum of the NR vectors x[r] (ranks in `mask`, ascending), scaled, in the vector's dtype.  mask == 0 -> zeros.
+template <int NR>
+__device__ __forceinline__ uint4 combine_vec(int dt, const uint4 (&x)[NR], uint32_t mask, float s, bool do_scale) {
+  const bool all = mask == (1u << NR) - 1u;
+  if (dt == MB_DT_F32) {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    bool first = true;
+#pragma unroll
+    for (int r = 0; r < NR; ++r) {
+      if (!all && !(mask & (1u << r))) continue;
+      const float4 y = make_float4(__uint_as_float(x[r].x), __uint_as_float(x[r].y), __uint_as_float(x[r].z),
+                                   __uint_as_float(x[r].w));
+      if (first) acc = y;
+      else add4(acc, y);
+      first = false;
+    }
+    acc = scale_vec(acc, s, do_scale);
+    return make_uint4(__float_as_uint(acc.x), __float_as_uint(acc.y), __float_as_uint(acc.z), __float_as_uint(acc.w));
+  }
+  float acc[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+  bool first = true;
+#pragma unroll
+  for (int r = 0; r < NR; ++r) {
+    if (!all && !(mask & (1u << r))) continue;
+    float y[8];
+    widen8(dt, x[r], y);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = first ? y[j] : __fadd_rn(acc[j], y[j]);
+    first = false;
+  }
+  if (do_scale) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = __fmul_rn(acc[j], s);
+  }
+  return narrow8(dt, acc);
+}
+
+// Reduce U vectors: all U*NR peer loads in flight before the first add (every rank contributes), or only the loads of
+// the ranks in `mask` (skipping ranks: rare).  Results are already scaled and rounded to the vector's dtype.
+template <int NR, int U>
+__device__ __forceinline__ void reduce_vecs_seg(const ArSegParams& p, uint32_t mask, const uint64_t (&v)[U],
+                                                float s, bool do_scale, uint4 (&out)[U]) {
+  const uint4* const* stage = reinterpret_cast<const uint4* const*>(p.b.stage);
+  uint4 x[U][NR];
+  const bool all = mask == (1u << NR) - 1u;
+#pragma unroll
+  for (int k = 0; k < U; ++k)
+#pragma unroll
+    for (int r = 0; r < NR; ++r) x[k][r] = (all || (mask & (1u << r))) ? ld_peer_u4(stage[r] + v[k]) : make_uint4(0, 0, 0, 0);
+#pragma unroll
+  for (int k = 0; k < U; ++k) out[k] = combine_vec<NR>(seg_dtype(p.seg, v[k]), x[k], mask, s, do_scale);
+}
+
+// Byte-table destination: 16 B stores, or 2 B stores for a tensor's tail / an unaligned tensor.
+__device__ __forceinline__ void scatter_bytes(const TensorTable& tb, uint64_t v, const uint4& r, uint32_t& cur) {
+  seek_tensor(tb, (uint32_t)v, cur);
+  const uint64_t within = (v - tb.off[cur]) * 16;
+  const uint64_t nbytes = tb.numel[cur];
+  if (within >= nbytes) return;  // padding-only vector (empty tensor)
+  const uint64_t valid = nbytes - within;
+  char* d = reinterpret_cast<char*>(tb.ptr[cur]) + within;
+  if (valid >= 16 && (reinterpret_cast<uintptr_t>(d) & 15u) == 0) {
+    st_u4(reinterpret_cast<uint4*>(d), r);
+  } else {
+    const uint16_t* h = reinterpret_cast<const uint16_t*>(&r);
+    const int nh = valid >= 16 ? 8 : (int)(valid >> 1);
+    for (int i = 0; i < nh; ++i) reinterpret_cast<uint16_t*>(d)[i] = h[i];
+  }
+}
+
+struct SinkB {
+  TensorTable tb;
+  uint4* flat;
+  uint32_t cur;
+  __device__ __forceinline__ void put(uint64_t v, const uint4& r) {
+    if (flat) st_u4(flat + v, r);
+    else scatter_bytes(tb, v, r, cur);
+  }
+};
+
+__device__ __forceinline__ SinkB make_sink_b(const ArParams& p, uint8_t* smem) {
+  SinkB s;
+  s.cur = 0;
+  if (p.ntensors == 0) {
+    s.flat = reinterpret_cast<uint4*>(p.flat_dst);
+    s.tb = TensorTable{nullptr, nullptr, nullptr, 0};
+  } else {
+    s.flat = nullptr;
+    s.tb = load_table(smem, p.dst_tab, p.ntensors);
+  }
+  return s;
+}
+
+template <int NR, int U>
+__global__ void __launch_bounds__(kArThreads, 1) ar_oneshot_seg_kernel(const __grid_constant__ ArSegParams sp) {
+  extern __shared__ __align__(16) uint8_t dyn_smem[];
+  __shared__ mb_ar_hdr s_total;
+  __shared__ uint32_t s_mask;
+  const ArParams& p = sp.b;
+  SinkB sink = make_sink_b(p, dyn_smem);
+  if (!reduce_prologue(p, &s_total, &s_mask)) return;
+  const uint32_t mask = s_mask;
+  const mb_ar_hdr tot = s_total;
+  const bool do_scale = p.scale && tot.num_gradients != 0;
+  const float s = reduce_scale(p, tot);
+  const uint32_t nthr = blockDim.x;
+  const uint64_t kChunk = (uint64_t)U * nthr;
+  for (uint64_t base = (uint64_t)blockIdx.x * kChunk; base < p.total_vec; base += (uint64_t)gridDim.x * kChunk) {
+    if (base + kChunk <= p.total_vec && !p.force_u1) {
+      uint64_t v[U];
+      uint4 r[U];
+#pragma unroll
+      for (int k = 0; k < U; ++k) v[k] = base + (uint64_t)k * nthr + threadIdx.x;
+      reduce_vecs_seg<NR, U>(sp, mask, v, s, do_scale, r);
+#pragma unroll
+      for (int k = 0; k < U; ++k) sink.put(v[k], r[k]);
+    } else {
+      const uint64_t cend = min(base + kChunk, p.total_vec);
+      for (uint64_t v0 = base + threadIdx.x; v0 < cend; v0 += nthr) {
+        uint64_t v[1] = {v0};
+        uint4 r[1];
+        reduce_vecs_seg<NR, 1>(sp, mask, v, s, do_scale, r);
+        sink.put(v0, r[0]);
+      }
+    }
+  }
+  write_result(p, tot);
+}
+
+// Same phases as ar_twoshot_kernel: the reduce-scatter stores the ROUNDED values, the all-gather and the local copy
+// move bytes.
+template <int NR, int U>
+__global__ void __launch_bounds__(kArThreads, 1) ar_twoshot_seg_kernel(const __grid_constant__ ArSegParams sp) {
+  extern __shared__ __align__(16) uint8_t dyn_smem[];
+  __shared__ mb_ar_hdr s_total;
+  __shared__ uint32_t s_mask;
+  const ArParams& p = sp.b;
+  SinkB sink = make_sink_b(p, dyn_smem);
+  if (!reduce_prologue(p, &s_total, &s_mask)) return;
+  const uint32_t mask = s_mask;
+  const mb_ar_hdr tot = s_total;
+  const bool do_scale = p.scale && tot.num_gradients != 0;
+  const float s = reduce_scale(p, tot);
+  const uint32_t nthr = blockDim.x;
+  const uint64_t kChunk = (uint64_t)U * nthr;
+  const uint64_t gstride = (uint64_t)gridDim.x * kChunk;
+  uint4* const* stage = reinterpret_cast<uint4* const*>(p.stage);
+  {
+    const uint64_t sbase = (uint64_t)p.rank * p.slice_vec;
+    const uint64_t slen = sbase < p.total_vec ? min(p.slice_vec, p.total_vec - sbase) : 0;
+    for (uint64_t cb = (uint64_t)blockIdx.x * kChunk; cb < slen; cb += gstride) {
+      if (cb + kChunk <= slen && !p.force_u1) {
+        uint64_t v[U];
+        uint4 r[U];
+#pragma unroll
+        for (int k = 0; k < U; ++k) v[k] = sbase + cb + (uint64_t)k * nthr + threadIdx.x;
+        reduce_vecs_seg<NR, U>(sp, mask, v, s, do_scale, r);
+#pragma unroll
+        for (int k = 0; k < U; ++k)
+#pragma unroll
+          for (int q = 0; q < NR; ++q) st_u4(stage[q] + v[k], r[k]);
+      } else {
+        const uint64_t cend = min(cb + kChunk, slen);
+        for (uint64_t j = cb + threadIdx.x; j < cend; j += nthr) {
+          uint64_t v[1] = {sbase + j};
+          uint4 r[1];
+          reduce_vecs_seg<NR, 1>(sp, mask, v, s, do_scale, r);
+#pragma unroll
+          for (int q = 0; q < NR; ++q) st_u4(stage[q] + v[0], r[0]);
+        }
+      }
+    }
+  }
+  if (!block_barrier(p, true)) {
+    report_failure(p);
+    return;
+  }
+  if (p.inplace) {
+    write_result(p, tot);
+    return;
+  }
+  const uint4* mine = stage[p.rank];
+#pragma unroll 1
+  for (int q = 0; q < NR; ++q) {
+    const uint64_t sbase = (uint64_t)q * p.slice_vec;
+    const uint64_t slen = sbase < p.total_vec ? min(p.slice_vec, p.total_vec - sbase) : 0;
+    for (uint64_t cb = (uint64_t)blockIdx.x * kChunk; cb < slen; cb += gstride) {
+      const uint64_t cend = min(cb + kChunk, slen);
+      if (cb + kChunk <= slen) {
+        uint4 x[U];
+#pragma unroll
+        for (int k = 0; k < U; ++k) x[k] = ld_peer_u4(mine + sbase + cb + (uint64_t)k * nthr + threadIdx.x);
+#pragma unroll
+        for (int k = 0; k < U; ++k) sink.put(sbase + cb + (uint64_t)k * nthr + threadIdx.x, x[k]);
+      } else {
+        for (uint64_t j = cb + threadIdx.x; j < cend; j += nthr) sink.put(sbase + j, ld_peer_u4(mine + sbase + j));
+      }
+    }
+  }
+  write_result(p, tot);
+}
+
+using ArSegKernel = void (*)(const ArSegParams);
+
+template <int NR, int U>
+ArSegKernel pick_seg(bool twoshot) {
+  return twoshot ? (ArSegKernel)ar_twoshot_seg_kernel<NR, U> : (ArSegKernel)ar_oneshot_seg_kernel<NR, U>;
+}
+
+// Same U x NR table as pick_unroll, but only the reachable pairs are instantiated: eight fp32 accumulators per
+// half-width vector make the unreachable ones (e.g. U=8 at NR=8) spill at 512 threads.
+template <int NR>
+ArSegKernel pick_unroll_seg(bool twoshot, int unroll) {
+  if constexpr (NR <= 2) {
+    if (unroll >= 8) return pick_seg<NR, 8>(twoshot);
+  }
+  if constexpr (NR <= 4) {
+    if (unroll >= 4) return pick_seg<NR, 4>(twoshot);
+  }
+  if (unroll >= 2) return pick_seg<NR, 2>(twoshot);
+  return pick_seg<NR, 1>(twoshot);
+}
+
+ArSegKernel kernel_for_seg(int world, bool twoshot, int want_unroll, int* unroll_out) {
+  int u = want_unroll >= 8 && world <= 2 ? 8 : want_unroll >= 4 && world <= 4 ? 4 : want_unroll >= 2 ? 2 : 1;
+  *unroll_out = u;
+  switch (world) {
+    case 1: return pick_unroll_seg<1>(twoshot, u);
+    case 2: return pick_unroll_seg<2>(twoshot, u);
+    case 3: return pick_unroll_seg<3>(twoshot, u);
+    case 4: return pick_unroll_seg<4>(twoshot, u);
+    case 5: return pick_unroll_seg<5>(twoshot, u);
+    case 6: return pick_unroll_seg<6>(twoshot, u);
+    case 7: return pick_unroll_seg<7>(twoshot, u);
+    case 8: return pick_unroll_seg<8>(twoshot, u);
+  }
+  return nullptr;
+}
+
+// K-A1 for mixed lists: staging (=|+=) sources, per 16 B vector; += rounds in the dtype (ATen's add_ on bf16 / fp16
+// computes in fp32 and rounds once).
+__global__ void __launch_bounds__(kArThreads) ar_stage_seg_kernel(const __grid_constant__ StageSegParams sp) {
+  extern __shared__ __align__(16) uint8_t dyn_smem[];
+  const StageParams& p = sp.b;
+  const TensorTable tb = load_table(dyn_smem, p.tab, p.ntensors);
+  __syncthreads();
+  const uint64_t per_block = (p.total_vec + gridDim.x - 1) / gridDim.x;
+  const uint64_t begin = (uint64_t)blockIdx.x * per_block;
+  const uint64_t end = min(begin + per_block, p.total_vec);
+  uint32_t cur = 0;
+  for (uint64_t v = begin + threadIdx.x; v < end; v += kArThreads) {
+    seek_tensor(tb, (uint32_t)v, cur);
+    const uint64_t within = (v - tb.off[cur]) * 16;
+    const uint64_t nbytes = tb.numel[cur];
+    uint4 g = make_uint4(0, 0, 0, 0);
+    if (within < nbytes) {
+      char* s = reinterpret_cast<char*>(tb.ptr[cur]) + within;
+      const uint64_t valid = nbytes - within;
+      if (valid >= 16 && (reinterpret_cast<uintptr_t>(s) & 15u) == 0) {
+        g = *reinterpret_cast<const uint4*>(s);
+        if (p.zero_src) *reinterpret_cast<uint4*>(s) = make_uint4(0, 0, 0, 0);
+      } else {
+        uint16_t* h = reinterpret_cast<uint16_t*>(&g);
+        const int nh = valid >= 16 ? 8 : (int)(valid >> 1);
+        for (int i = 0; i < nh; ++i) {
+          h[i] = reinterpret_cast<const uint16_t*>(s)[i];
+          if (p.zero_src) reinterpret_cast<uint16_t*>(s)[i] = 0;
+        }
+      }
+    }
+    uint4* d = reinterpret_cast<uint4*>(p.staging) + v;
+    if (p.accumulate) {
+      const uint4 a = *d;
+      const int dt = seg_dtype(sp.seg, v);
+      if (dt == MB_DT_F32) {
+        g = make_uint4(__float_as_uint(__fadd_rn(__uint_as_float(a.x), __uint_as_float(g.x))),
+                       __float_as_uint(__fadd_rn(__uint_as_float(a.y), __uint_as_float(g.y))),
+                       __float_as_uint(__fadd_rn(__uint_as_float(a.z), __uint_as_float(g.z))),
+                       __float_as_uint(__fadd_rn(__uint_as_float(a.w), __uint_as_float(g.w))));
+      } else {
+        float fa[8], fg[8];
+        widen8(dt, a, fa);
+        widen8(dt, g, fg);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) fa[j] = __fadd_rn(fa[j], fg[j]);
+        g = narrow8(dt, fa);
+      }
+    }
+    *d = g;
+  }
+}
+
 // ---- host helpers ------------------------------------------------------------------------------------------------
 
 constexpr int kBufs = MB_AR_BUFS_PER_SLOT;
@@ -742,7 +1108,7 @@ uint64_t flat_layout(const uint64_t* numel, int n) {
 int sync_table(mb_ar_ctx* ctx, int which, const void* const* ptrs, const uint64_t* numel, int n, uint64_t* total_out,
                cudaStream_t stream) {
   auto& cache = ctx->tab_host[which];
-  bool same = cache.size() == (size_t)n;
+  bool same = cache.size() == (size_t)n && !ctx->tab_bytes[which];
   uint64_t off = 0;
   for (int i = 0; i < n; ++i) {
     if (same) {
@@ -753,6 +1119,7 @@ int sync_table(mb_ar_ctx* ctx, int which, const void* const* ptrs, const uint64_
   }
   *total_out = off;
   if (same) return MB_OK;
+  ctx->tab_bytes[which] = false;
   cache.resize(n);
   off = 0;
   for (int i = 0; i < n; ++i) {
@@ -765,6 +1132,69 @@ int sync_table(mb_ar_ctx* ctx, int which, const void* const* ptrs, const uint64_
     MB_CUDA(cudaMemcpyAsync(ctx->tab_dev[which], cache.data(), (size_t)n * sizeof(TensorEnt), cudaMemcpyHostToDevice,
                             stream));
   }
+  return MB_OK;
+}
+
+// mb_ar_layout: dtype runs in the order fp32, bf16, fp16, list order inside a run, every tensor 16 B aligned.
+int layout_ex(const uint64_t* numel, const int32_t* dtype, int n, uint64_t* off, uint64_t* total, mb_ar_segment* segs) {
+  static const int32_t kOrder[3] = {MB_DT_F32, MB_DT_BF16, MB_DT_F16};
+  uint64_t at = 0;
+  int nseg = 0;
+  for (int32_t d : kOrder) {
+    const uint64_t begin = at, esize = d == MB_DT_F32 ? 4 : 2;
+    for (int i = 0; i < n; ++i) {
+      if (dtype[i] != d) continue;
+      if (off) off[i] = at;
+      at += (numel[i] * esize + 15) & ~15ull;
+    }
+    if (at > begin) {
+      if (segs) segs[nseg] = mb_ar_segment{begin, at, d, 0};
+      ++nseg;
+    }
+  }
+  if (total) *total = at;
+  return nseg;
+}
+
+SegInfo seg_info(const mb_ar_segment* segs, int nseg) {
+  SegInfo si;
+  for (int k = 0; k < 3; ++k) {
+    si.end[k] = k < nseg ? segs[k].end / 16 : ~0ull;
+    si.dt[k] = k < nseg ? segs[k].dtype : (nseg ? segs[nseg - 1].dtype : MB_DT_F32);
+  }
+  return si;
+}
+
+// Validates a dtype array; *all_f32 = every tensor is fp32 (the list then runs the fp32 entry points unchanged).
+int check_dtypes(const char* fn, const int32_t* dtype, int n, bool* all_f32) {
+  *all_f32 = true;
+  for (int i = 0; i < n; ++i) {
+    MB_CHECK_ARG(dtype[i] == MB_DT_F32 || dtype[i] == MB_DT_BF16 || dtype[i] == MB_DT_F16,
+                 "%s: tensor %d has dtype %d; supported: MB_DT_F32, MB_DT_BF16, MB_DT_F16", fn, i, (int)dtype[i]);
+    if (dtype[i] != MB_DT_F32) *all_f32 = false;
+  }
+  return MB_OK;
+}
+
+// Byte-table variant of sync_table for mixed lists: entries in layout (offset) order, {ptr, byte offset / 4, bytes}.
+int sync_table_bytes(mb_ar_ctx* ctx, int which, const void* const* ptrs, const uint64_t* numel, const int32_t* dtype,
+                     int n, const uint64_t* off, cudaStream_t stream) {
+  std::vector<TensorEnt> ents;
+  ents.reserve(n);
+  for (int32_t d : {MB_DT_F32, MB_DT_BF16, MB_DT_F16})
+    for (int i = 0; i < n; ++i)
+      if (dtype[i] == d)
+        ents.push_back(TensorEnt{reinterpret_cast<uint64_t>(ptrs[i]), off[i] / 4, numel[i] * (d == MB_DT_F32 ? 4 : 2)});
+  auto& cache = ctx->tab_host[which];
+  bool same = ctx->tab_bytes[which] && cache.size() == ents.size();
+  for (size_t i = 0; same && i < ents.size(); ++i)
+    same = cache[i].ptr == ents[i].ptr && cache[i].off == ents[i].off && cache[i].numel == ents[i].numel;
+  if (same) return MB_OK;
+  cache.swap(ents);
+  ctx->tab_bytes[which] = true;
+  if (n > 0)
+    MB_CUDA(cudaMemcpyAsync(ctx->tab_dev[which], cache.data(), (size_t)n * sizeof(TensorEnt), cudaMemcpyHostToDevice,
+                            stream));
   return MB_OK;
 }
 
@@ -800,15 +1230,28 @@ int ensure_dyn_smem(const void* fn, size_t bytes) {
 
 size_t table_bytes(uint32_t n) { return (size_t)n * (8 + 8 + 4); }
 
-// Shared by mb_ar_allreduce (ungated: in-kernel per-block barrier) and mb_ar_reduce_gated (K-A0 + barrier-free reduce).
+// A mixed-dtype round whose byte table (tab_dev[1]) is already uploaded: see launch_reduce.
+struct SegLaunch {
+  uint64_t total_vec;
+  uint32_t ntab;  // 0: the result goes to `flat`
+  void* flat;
+  SegInfo info;
+};
+
+// Shared by mb_ar_allreduce (ungated: in-kernel per-block barrier) and mb_ar_reduce_gated (K-A0 + barrier-free reduce),
+// and by their _ex variants for lists with bf16 / fp16 segments (seg != nullptr: dst / numel / flat_* are unused).
 int launch_reduce(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, float* const* dst, const uint64_t* numel,
                   int ntensors, float* flat_dst, uint64_t flat_numel, int scale, int algo, uint32_t timeout_ms,
-                  bool gated, uint64_t min_batch, cudaStream_t stream) {
+                  bool gated, uint64_t min_batch, cudaStream_t stream, const SegLaunch* seg = nullptr) {
   uint64_t total = 0;
   uint32_t ntab = 0;
   float* flat_sink = nullptr;
   const bool timed_round = gated;
-  if (dst) {
+  if (seg) {
+    total = seg->total_vec * 4;
+    ntab = seg->ntab;
+    flat_sink = static_cast<float*>(seg->flat);
+  } else if (dst) {
     MB_CHECK_ARG(numel != nullptr, "mb_ar_allreduce: numel is null");
     MB_CHECK_ARG(ntensors >= 1 && ntensors <= kArMaxTensors, "mb_ar_allreduce: ntensors %d not in [1,%d]", ntensors,
                  kArMaxTensors);
@@ -931,7 +1374,10 @@ int launch_reduce(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, float* cons
   if (!env_threads)
     while (threads > 128 && chunks(threads, want_unroll) < max_grid) threads >>= 1;
   int unroll = 1;
-  ArKernel k = kernel_for(ctx->world, twoshot, want_unroll, &unroll);
+  ArKernel k = nullptr;
+  ArSegKernel ks = nullptr;
+  if (seg) ks = kernel_for_seg(ctx->world, twoshot, want_unroll, &unroll);
+  else k = kernel_for(ctx->world, twoshot, want_unroll, &unroll);
   const uint64_t chunk = (uint64_t)threads * unroll;
   uint64_t want = (work_vec + chunk - 1) / chunk;
   if (want == 0) want = 1;
@@ -939,9 +1385,18 @@ int launch_reduce(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, float* cons
   p.inplace = (twoshot && flat_sink != nullptr && flat_sink == p.stage[ctx->rank]) ? 1 : 0;
   const uint32_t grid = (uint32_t)std::min<uint64_t>(want, max_grid);
   const size_t smem = table_bytes(ntab);
-  int rc = ensure_dyn_smem(reinterpret_cast<const void*>(k), smem);
-  if (rc) return rc;
-  k<<<grid, threads, smem, stream>>>(p);
+  if (seg) {
+    int rc = ensure_dyn_smem(reinterpret_cast<const void*>(ks), smem);
+    if (rc) return rc;
+    ArSegParams sp;
+    sp.b = p;
+    sp.seg = seg->info;
+    ks<<<grid, threads, smem, stream>>>(sp);
+  } else {
+    int rc = ensure_dyn_smem(reinterpret_cast<const void*>(k), smem);
+    if (rc) return rc;
+    k<<<grid, threads, smem, stream>>>(p);
+  }
   MB_CUDA(cudaGetLastError());
   if (timed) {
     MB_CUDA(cudaEventRecord(ctx->ev[slot][2], stream));
@@ -1250,6 +1705,137 @@ int mb_ar_reduce_gated(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, uint64
   DeviceGuard g(ctx->device);
   return launch_reduce(ctx, slot, my_hdr, dst, numel, ntensors, flat_dst, flat_numel, scale_by_num_gradients, algo,
                        timeout_ms, /*gated=*/true, min_batch_size, static_cast<cudaStream_t>(stream_));
+}
+
+int mb_ar_layout(const uint64_t* numel, const int32_t* dtype, int ntensors, uint64_t* offset_bytes,
+                 uint64_t* total_bytes, mb_ar_segment* segments) {
+  MB_CHECK_ARG(ntensors >= 0 && (ntensors == 0 || (numel && dtype)), "mb_ar_layout: null argument");
+  bool all_f32 = true;
+  int rc = check_dtypes("mb_ar_layout", dtype, ntensors, &all_f32);
+  if (rc) return rc;
+  return layout_ex(numel, dtype, ntensors, offset_bytes, total_bytes, segments);
+}
+
+int mb_ar_stage_ex(mb_ar_ctx* ctx, int slot, const void* const* grads, const uint64_t* numel, const int32_t* dtype,
+                   int ntensors, int accumulate, int zero_src, mb_stream_t stream_) {
+  MB_CHECK_ARG(ctx && grads && numel && dtype, "mb_ar_stage_ex: null argument");
+  MB_CHECK_ARG(slot >= 0 && slot < ctx->nslots, "mb_ar_stage_ex: slot %d out of range", slot);
+  MB_CHECK_ARG(ntensors >= 1 && ntensors <= kArMaxTensors, "mb_ar_stage_ex: ntensors %d not in [1,%d]", ntensors,
+               kArMaxTensors);
+  bool all_f32 = true;
+  int rc = check_dtypes("mb_ar_stage_ex", dtype, ntensors, &all_f32);
+  if (rc) return rc;
+  if (all_f32)
+    return mb_ar_stage(ctx, slot, reinterpret_cast<const float* const*>(grads), numel, ntensors, accumulate, zero_src,
+                       stream_);
+  std::vector<uint64_t> off(ntensors);
+  mb_ar_segment segs[3];
+  uint64_t total = 0;
+  const int nseg = layout_ex(numel, dtype, ntensors, off.data(), &total, segs);
+  MB_CHECK_ARG(total <= ctx->max_bytes, "mb_ar_stage_ex: %llu bytes exceed the context's max_bytes %llu",
+               (unsigned long long)total, (unsigned long long)ctx->max_bytes);
+  std::lock_guard<std::mutex> l(ctx->mu);
+  DeviceGuard g(ctx->device);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  rc = sync_table_bytes(ctx, 0, grads, numel, dtype, ntensors, off.data(), stream);
+  if (rc) return rc;
+  if (total == 0) return 0;
+  StageSegParams sp;
+  sp.b.staging = ring_buffer(ctx, ctx->staging, slot, 0);
+  sp.b.tab = ctx->tab_dev[0];
+  sp.b.ntensors = (uint32_t)ntensors;
+  sp.b.accumulate = accumulate;
+  sp.b.zero_src = zero_src;
+  sp.b.total_vec = total / 16;
+  sp.seg = seg_info(segs, nseg);
+  const int sms = sm_count(ctx->device);
+  if (sms <= 0) return MB_ECUDA;
+  const uint64_t want = (sp.b.total_vec + kArThreads - 1) / kArThreads;
+  const uint32_t grid = (uint32_t)std::min<uint64_t>(want, (uint64_t)sms * 4);
+  const size_t smem = table_bytes(sp.b.ntensors);
+  rc = ensure_dyn_smem(reinterpret_cast<const void*>(ar_stage_seg_kernel), smem);
+  if (rc) return rc;
+  ar_stage_seg_kernel<<<grid, kArThreads, smem, stream>>>(sp);
+  MB_CUDA(cudaGetLastError());
+  return 1;
+}
+
+// mb_ar_allreduce_ex / mb_ar_reduce_gated_ex; the caller holds ctx->mu and the device guard.
+static int reduce_ex_locked(const char* fn, mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, void* const* dst,
+                            const uint64_t* numel, const int32_t* dtype, int ntensors, void* flat_dst,
+                            uint64_t flat_bytes, int scale, int algo, uint32_t timeout_ms, bool gated,
+                            uint64_t min_batch, cudaStream_t stream) {
+  std::vector<uint64_t> off(ntensors);
+  mb_ar_segment segs[3];
+  uint64_t total = 0;
+  const int nseg = layout_ex(numel, dtype, ntensors, off.data(), &total, segs);
+  bool all_f32 = nseg == 0 || (nseg == 1 && segs[0].dtype == MB_DT_F32);
+  for (int i = 0; i < ntensors; ++i) all_f32 = all_f32 && dtype[i] == MB_DT_F32;
+  if (!dst) {
+    MB_CHECK_ARG(flat_dst != nullptr, "%s: neither dst nor flat_dst given", fn);
+    MB_CHECK_ARG(flat_bytes == total, "%s: flat_bytes %llu != layout size %llu", fn, (unsigned long long)flat_bytes,
+                 (unsigned long long)total);
+    MB_CHECK_ARG((reinterpret_cast<uintptr_t>(flat_dst) & 15u) == 0, "%s: flat_dst is not 16 B aligned", fn);
+  }
+  if (all_f32) {
+    // exactly what mb_ar_allreduce / mb_ar_reduce_gated run for this list
+    if (dst)
+      return launch_reduce(ctx, slot, my_hdr, reinterpret_cast<float* const*>(dst), numel, ntensors, nullptr, 0, scale,
+                           algo, timeout_ms, gated, min_batch, stream);
+    return launch_reduce(ctx, slot, my_hdr, nullptr, nullptr, 0, static_cast<float*>(flat_dst), total / 4, scale, algo,
+                         timeout_ms, gated, min_batch, stream);
+  }
+  MB_CHECK_ARG(total <= ctx->max_bytes, "%s: %llu bytes exceed the context's max_bytes %llu", fn,
+               (unsigned long long)total, (unsigned long long)ctx->max_bytes);
+  SegLaunch sl;
+  sl.total_vec = total / 16;
+  sl.ntab = 0;
+  sl.flat = flat_dst;
+  sl.info = seg_info(segs, nseg);
+  if (dst) {
+    int rc = sync_table_bytes(ctx, 1, dst, numel, dtype, ntensors, off.data(), stream);
+    if (rc) return rc;
+    sl.ntab = (uint32_t)ntensors;
+    sl.flat = nullptr;
+  }
+  return launch_reduce(ctx, slot, my_hdr, nullptr, nullptr, 0, nullptr, 0, scale, algo, timeout_ms, gated, min_batch,
+                       stream, &sl);
+}
+
+static int reduce_ex_args(const char* fn, mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, const uint64_t* numel,
+                          const int32_t* dtype, int ntensors) {
+  MB_CHECK_ARG(ctx && my_hdr && numel && dtype, "%s: null argument", fn);
+  MB_CHECK_ARG(slot >= 0 && slot < ctx->nslots, "%s: slot %d out of range", fn, slot);
+  MB_CHECK_ARG(ntensors >= 1 && ntensors <= kArMaxTensors, "%s: ntensors %d not in [1,%d]", fn, ntensors,
+               kArMaxTensors);
+  bool all_f32 = true;
+  return check_dtypes(fn, dtype, ntensors, &all_f32);
+}
+
+int mb_ar_allreduce_ex(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, void* const* dst, const uint64_t* numel,
+                       const int32_t* dtype, int ntensors, void* flat_dst, uint64_t flat_bytes,
+                       int scale_by_num_gradients, int algo, uint32_t timeout_ms, mb_stream_t stream_) {
+  int rc = reduce_ex_args("mb_ar_allreduce_ex", ctx, slot, my_hdr, numel, dtype, ntensors);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> l(ctx->mu);
+  DeviceGuard g(ctx->device);
+  rc = reduce_ex_locked("mb_ar_allreduce_ex", ctx, slot, my_hdr, dst, numel, dtype, ntensors, flat_dst, flat_bytes,
+                        scale_by_num_gradients, algo, timeout_ms, /*gated=*/false, 0, static_cast<cudaStream_t>(stream_));
+  if (rc >= 0) ctx->parity[slot] = (ctx->parity[slot] + 1) % kBufs;
+  return rc;
+}
+
+int mb_ar_reduce_gated_ex(mb_ar_ctx* ctx, int slot, const mb_ar_hdr* my_hdr, uint64_t min_batch_size, void* const* dst,
+                          const uint64_t* numel, const int32_t* dtype, int ntensors, void* flat_dst,
+                          uint64_t flat_bytes, int scale_by_num_gradients, int algo, uint32_t timeout_ms,
+                          mb_stream_t stream_) {
+  int rc = reduce_ex_args("mb_ar_reduce_gated_ex", ctx, slot, my_hdr, numel, dtype, ntensors);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> l(ctx->mu);
+  DeviceGuard g(ctx->device);
+  return reduce_ex_locked("mb_ar_reduce_gated_ex", ctx, slot, my_hdr, dst, numel, dtype, ntensors, flat_dst, flat_bytes,
+                          scale_by_num_gradients, algo, timeout_ms, /*gated=*/true, min_batch_size,
+                          static_cast<cudaStream_t>(stream_));
 }
 
 int mb_ar_round_times(mb_ar_ctx* ctx, int slot, float* gate_us, float* reduce_us) {
